@@ -7,6 +7,8 @@ views, CFG batch 2, bf16, 50-step DDIM schedule).
 
 One "step" = one iteration of the reference loop models/pano/PanFusion.py:146-162: rotate, CFG-batched
 MultiViewBaseModel.forward (7 EPPA fusions), CFG combine, two DDIM updates. Prints ONE JSON line (rank 0).
+`--dump-outputs DIR` writes the view and panorama latents after the last timed step as DIR/<name>.npy (float32); the
+inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -140,6 +142,16 @@ def synthetic_inputs(wl, ctx_dim, device, sampler, seed=0):
     return out
 
 
+def dump_outputs(out_dir, latents, pano_latent):
+    """What the caller of the denoise loop receives after the last timed step: the view latents [1, m, 4, h, w] and the
+    panorama latent [1, 1, 4, H, W], as float32 .npy files."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in (("latents", latents), ("pano_latent", pano_latent)):
+        np.save(d / f"{name}.npy", t.detach().to("cpu", torch.float32).numpy())
+
+
 # ------------------------------------------------------------------------------------------------------
 # this repo's arm
 # ------------------------------------------------------------------------------------------------------
@@ -224,6 +236,8 @@ def run_b200(args):
         e1.record()
         torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *sampler.finish())
     if world > 1:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -535,24 +549,25 @@ def cpu_baseline(workload, budget_s=30.0):
 def run_reference(args):
     """`--impl reference`: the reference algorithm's own CPU path (oracle port; diffusers/xformers/kornia are not
     installable offline, SURVEY.md §8c) on the usable host cores, REAL steps of the benchmark workload: one warm-up
-    step, then as many timed steps as fit `--ref-budget` seconds (at least 2, at most --steps). `steps` / `warmup` in
-    the JSON line are the counts actually run. Rank 0 only."""
+    step, then --steps timed steps (about a minute each at C2). `steps` / `warmup` in the JSON line are the counts
+    actually run. Rank 0 only."""
     if int(os.environ.get("RANK", 0)) != 0:
         return
     wl = WORKLOADS[args.workload]
     cores = host_threads()
     loop = _OracleLoop(args.workload)
-    t_warm = loop.step()
-    n_timed = max(2, min(args.steps, int(args.ref_budget / max(t_warm, 1e-3))))
-    times = [loop.step() for _ in range(n_timed)]
-    per = sum(times) / n_timed
+    loop.step()
+    times = [loop.step() for _ in range(args.steps)]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, loop.lat, loop.pano)
+    per = sum(times) / args.steps
     val = round(1.0 / per, 5)
-    sample = (f"{n_timed} full denoise steps of this workload after 1 warm-up step (rotate + CFG-batched forward + combine "
+    sample = (f"{args.steps} full denoise steps of this workload after 1 warm-up step (rotate + CFG-batched forward + combine "
               f"+ 2 DDIM updates; reference algorithm via the oracle port, fp32, {cores} threads): "
               f"{', '.join(f'{t:.1f}' for t in times)} s; measured, not scaled")
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": val, "unit": "steps/s", "n_gpus": args.gpus,
-        "steps": n_timed, "warmup": 1, "ms_per_step": round(per * 1e3, 1), "higher_is_better": True,
+        "steps": args.steps, "warmup": 1, "ms_per_step": round(per * 1e3, 1), "higher_is_better": True,
         "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": wl["desc"], "views": wl["m"], "cfg_batch": 2, "pano_latent": list(wl["pano_hw"]),
                    "view_latent": list(wl["pers_hw"]), "weights": "synthetic SD-2 architecture"},
@@ -573,10 +588,12 @@ def main():
     ap.add_argument("--skip-micro", action="store_true", help="skip the isolated kernel rooflines")
     ap.add_argument("--skip-image", action="store_true", help="skip the cold / warm whole-image latency leg")
     ap.add_argument("--cpu-budget", type=float, default=30.0)
-    ap.add_argument("--ref-budget", type=float, default=240.0,
-                    help="--impl reference: seconds of TIMED reference steps (at least 2 steps are always run)")
     ap.add_argument("--profile-one-step", action="store_true", help="for ncu --profile-from-start off: profile one eager step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the latents of the last timed step as DIR/latents.npy and DIR/pano_latent.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

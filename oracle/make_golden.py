@@ -41,6 +41,15 @@ def _report(name, ref, mine):
     return err
 
 
+def round_mantissa(a: np.ndarray, bits: int = 15) -> np.ndarray:
+    """float32 rounded to nearest with `bits` of its 23 mantissa bits kept (relative error <= 2**-(bits + 1)). The low
+    mantissa bits of model outputs do not compress; dropping 8 of them keeps a fixture under 1 MB at 1.5e-5 of each
+    value, far below the 4e-3 / 2.5e-2 parity gates it is compared at."""
+    u = np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)
+    drop = 23 - bits
+    return ((u + np.uint32(1 << (drop - 1))) >> drop << drop).astype(np.uint32).view(np.float32)
+
+
 def golden_c2(ref):
     """BASELINE configs[1], the benchmarked configuration: SD-2 widths, 8 horizon views 64x64 + pano 64x128, the CFG
     pair (b = 2, prompts [null; text]) — ONE reference MultiViewBaseModel.forward (MVGenModel.py:38-297) on CPU."""
@@ -51,7 +60,7 @@ def golden_c2(ref):
     rs, rp_ = model_r(**inp)
     t1 = time.time()
     print(f"  [c2] reference forward {t1 - t0:.1f}s", flush=True)
-    np.savez_compressed(OUT / "mvgen_c2.npz", sample=rs.numpy(), pano_sample=rp_.numpy())
+    np.savez_compressed(OUT / "mvgen_c2.npz", sample=round_mantissa(rs.numpy()), pano_sample=round_mantissa(rp_.numpy()))
     model_o = synth.build_model(om.MultiViewBaseModel, cfg, seed=0)
     model_o.load_state_dict(model_r.state_dict())
     del model_r
